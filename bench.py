@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the NERRF AI hot path on B200 (driver contract).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): GraphSAGE-T edges/sec (+ MCTS rollouts/sec, reported under "mcts") on the
@@ -25,6 +25,11 @@ N > 1: weak scaling -- the graph grows to N x (1M nodes, 10M edges), 1-D edge-bl
 embedding exchange per layer fused into the layer kernel (nerrf_b200/dist.py).  Extra objects of the N>1 line:
 "trace_graph" (trace-structured graph, component-aware cuts), "cfg4" (BASELINE configs[3]: 10M / 100M strong-scaled
 over the N GPUs), "cfg5" (configs[4]: the streamed LockBit fleet trace end to end), "nvlink" (achieved GB/s).
+
+--dump-outputs DIR (single process): after the timed steps, what the forward returned in the LAST timed step, as float32
+.npy files: DIR/score.npy (the node score of every node, [N]) and DIR/h_sample.npy (the final embeddings of a fixed
+seeded sample of DUMP_ROWS nodes, [DUMP_ROWS, 128]; the full [N, 128] array is 512 MB).  The graph and the weights are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,10 +44,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # a run writes nothing into the tree, which may be read-only
 
 N_NODES, N_EDGES, F_IN, HIDDEN, LAYERS = 1_000_000, 10_000_000, 32, 128, 3
 MCTS_CFG = dict(A=1024, R=4096, D=50, T=64)
 GRAPH_SEED = 20250115
+DUMP_ROWS, DUMP_SEED = 32768, 0
 
 
 def algorithmic_bytes_layer(E, N, F, H=HIDDEN, s_rp=4):
@@ -119,6 +126,17 @@ def workload_config(n_gpus):
             "l2": "inputs exceed L2 (graph 0.2 GB + activations 0.5 GB/layer per GPU vs 126 MB); no flush"}
 
 
+def dump_rows(n):
+    """The rows of h written by --dump-outputs: a fixed seeded sample, sorted."""
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(n, DUMP_ROWS), replace=False))
+
+
+def write_outputs(out_dir, h_sample, score):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("h_sample", h_sample), ("score", score)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 # ------------------------------------------------------------------------------------------ oracle side (checker / CPU arm)
 def oracle_check(model, rowptr, col, ew, x, h_gpu, score_gpu, k=64):
     """The C/OpenMP oracle (oracle/c/sage_oracle.c) over the FULL graph on the host cores vs a GPU forward: every element
@@ -146,7 +164,8 @@ def oracle_check(model, rowptr, col, ew, x, h_gpu, score_gpu, k=64):
 
 
 def cpu_arm_forward(params, x, rowptr, col, ew, steps, warmup):
-    """Times the C/OpenMP oracle forward over the full graph with the thread count at which it runs fastest."""
+    """Times the C/OpenMP oracle forward over the full graph with the thread count at which it runs fastest.  Returns
+    (mean seconds, threads, the Forward holding the outputs of the last timed step)."""
     from oracle import c_sage
     f = c_sage.Forward(params, x, rowptr, col, ew)
     threads, _ = c_sage.tune_threads(f)
@@ -155,7 +174,7 @@ def cpu_arm_forward(params, x, rowptr, col, ew, steps, warmup):
     ts = []
     for _ in range(steps):
         t0 = time.perf_counter(); f.run(); ts.append(time.perf_counter() - t0)
-    return float(np.mean(ts)), threads
+    return float(np.mean(ts)), threads, f
 
 
 def run_reference(args):
@@ -178,7 +197,9 @@ def run_reference(args):
         rp, col, ew, x = (t.cpu().numpy() for t in gpu_synthetic_graph(N_NODES * n, N_EDGES * n, GRAPH_SEED, dev, relabel=True))
         torch.cuda.empty_cache()
     params = S.make_params(F_IN, HIDDEN, LAYERS, seed=1)
-    dt, threads = cpu_arm_forward(params, x, rp, col, ew, args.steps, max(args.warmup, 1))
+    dt, threads, f = cpu_arm_forward(params, x, rp, col, ew, args.steps, max(args.warmup, 1))
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, f.h[dump_rows(f.N)], f.score)
     E = int(col.shape[0])
     eps = E / dt
     sample = f"the full {LAYERS}-layer forward over the whole graph ({E} edges, {rp.shape[0] - 1} nodes), {args.steps} steps"
@@ -254,10 +275,14 @@ def run_single(args, dev, local_rank):
     torch.cuda.synchronize()
     t_start.record()
     for i in range(K):
-        step(i)
+        h_last, score_last = step(i)
     t_end.record()
     torch.cuda.synchronize()
     clocks = sampler.result()
+    if args.dump_outputs:
+        rows = torch.from_numpy(dump_rows(N)).to(dev)
+        write_outputs(args.dump_outputs, h_last.index_select(0, rows).cpu().numpy(), score_last.cpu().numpy())
+        del rows
     total_ms = t_start.elapsed_time(t_end)
     layer_ms = np.array([[ev[i][l].elapsed_time(ev[i][l + 1]) for l in range(LAYERS)] for i in range(K)])
     ms_per_step = total_ms / K
@@ -341,7 +366,7 @@ def run_single(args, dev, local_rank):
     cpu = None
     if not args.no_cpu_baseline:
         from oracle import sage_ref as S
-        dt, th = cpu_arm_forward(S.make_params(F_IN, HIDDEN, LAYERS, seed=1), g.x, g.rowptr, g.col, g.ew, 3, 1)
+        dt, th, _ = cpu_arm_forward(S.make_params(F_IN, HIDDEN, LAYERS, seed=1), g.x, g.rowptr, g.col, g.ew, 3, 1)
         cpu = {"value": E / dt, "unit": "edges/s", "cores": th, "kind": "port", "seconds": dt,
                "sample": f"oracle/c/sage_oracle.c (C + OpenMP), the full {LAYERS}-layer forward over the whole graph ({E} edges), mean of 3, "
                          f"thread count auto-tuned (host exposes {os.cpu_count()} logical CPUs)"}
@@ -779,7 +804,14 @@ def main():
                     help="N>1: per-layer embedding exchange: p2p = fused into the layer kernel (epilogue stores to "
                          "peer-mapped buffers over NVLink, only the rows a peer references); p2p-all = same, every row "
                          "to every peer; multicast = NVSwitch multimem.st; allgather / broadcast / allreduce = NCCL")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last one to DIR as float32 .npy (see the module "
+                         "docstring); single process only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs needs a single-process run")
     if args.impl == "reference":
         run_reference(args)
     else:

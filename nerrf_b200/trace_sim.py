@@ -4,8 +4,8 @@ Schema (keys / event names / phases) follows benchmarks/m1/scripts/sim_lockbit_m
 the shipped fixtures benchmarks/m{0,1}/results/*_trace.jsonl: timestamp (ISO), event, path,
 size, pid, phase, file_type; phases reconnaissance -> preparation (file_created) -> attack
 (file_encrypt_start on x.dat, file_encrypt_complete on x.lockbit3) -> ransom note.
-Used for tests and for the cfg-5 style end-to-end example; the real m0/m1 traces are read from
-the reference checkout when it is present (tests/golden/make_golden.py).
+Used for tests and for the cfg-5 style end-to-end example; the real m0/m1 traces are stored under
+tests/golden/ (m{0,1}_trace.jsonl).
 """
 from __future__ import annotations
 

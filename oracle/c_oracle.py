@@ -1,11 +1,14 @@
 """ctypes wrapper of the C restatement of the planner oracle (oracle/c/planner_oracle.c) -- TEST INFRASTRUCTURE.
 
-Built on demand with gcc into oracle/_build/ (git-ignored).  Used by tests/test_oracle_c.py to pin the numpy
-oracle bit for bit against a second, independent implementation, and by bench.py as the all-host-cores CPU
-baseline of the MCTS half of the metric.  Never imported by the product (nerrf_b200/)."""
+Built by build() with gcc into oracle/_build/ (git-ignored); when that library is missing or stale, lib() compiles it
+into a temporary directory that is removed once the library is loaded, so a run never writes into the tree.  Used by
+tests/test_oracle_c.py to pin the numpy oracle bit for bit against a second, independent implementation, and by
+bench.py as the all-host-cores CPU baseline of the MCTS half of the metric.  Never imported by the product
+(nerrf_b200/)."""
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -19,20 +22,29 @@ LIB = os.path.join(OUT_DIR, "libplanner_oracle.so")
 _lib = None
 
 
-def build(force=False):
-    os.makedirs(OUT_DIR, exist_ok=True)
-    if force or not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(SRC):
-        cmd = ["gcc", "-O2", "-fopenmp", "-ffp-contract=off", "-fno-fast-math", "-shared", "-fPIC", SRC, "-o", LIB, "-lm"]
+def _stale(out):
+    return not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(SRC)
+
+
+def build(force=False, out_dir=OUT_DIR):
+    os.makedirs(out_dir, exist_ok=True)
+    out = os.path.join(out_dir, os.path.basename(LIB))
+    if force or _stale(out):
+        cmd = ["gcc", "-O2", "-fopenmp", "-ffp-contract=off", "-fno-fast-math", "-shared", "-fPIC", SRC, "-o", out, "-lm"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("gcc failed on the C oracle:\n" + r.stdout + r.stderr)
-    return LIB
+    return out
 
 
 def lib():
     global _lib
     if _lib is None:
-        h = C.CDLL(build())
+        if _stale(LIB):
+            with tempfile.TemporaryDirectory(prefix="nerrf_planner_oracle_") as d:
+                h = C.CDLL(build(out_dir=d))
+        else:
+            h = C.CDLL(LIB)
         h.nerrf_oracle_mcts.restype = C.c_int
         _lib = h
     return _lib

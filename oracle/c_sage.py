@@ -6,13 +6,14 @@ Two uses, both on the checker side of the fence:
   * bench.py: the all-host-cores CPU arm (`--impl reference`, `cpu_baseline`) over the FULL graph.
 Never imported by the product (nerrf_b200/).
 
-Built on demand with gcc -O3 -march=native into oracle/_build/.  The file name carries a hash of this host's CPU
-flags, so a library built in the authoring container is not reused on a GPU box with a different CPU (it is
-rebuilt there in about a second; gcc is part of the image)."""
+Built by build() with gcc -O3 -march=native into oracle/_build/.  The file name carries a hash of this host's CPU
+flags, so a library built on another host is not reused: lib() then compiles it (about a second) into a temporary
+directory that is removed once the library is loaded, so a run never writes into the tree, which may be read-only."""
 import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -33,14 +34,18 @@ def _cpu_tag():
     return "generic"
 
 
-def lib_path():
-    return os.path.join(OUT_DIR, f"libsage_oracle_{_cpu_tag()}.so")
+def lib_path(out_dir=OUT_DIR):
+    return os.path.join(out_dir, f"libsage_oracle_{_cpu_tag()}.so")
 
 
-def build(force=False):
-    os.makedirs(OUT_DIR, exist_ok=True)
-    out = lib_path()
-    if force or not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(SRC):
+def _stale(out):
+    return not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(SRC)
+
+
+def build(force=False, out_dir=OUT_DIR):
+    os.makedirs(out_dir, exist_ok=True)
+    out = lib_path(out_dir)
+    if force or _stale(out):
         base = ["gcc", "-O3", "-fopenmp", "-fno-fast-math", "-shared", "-fPIC", SRC, "-lm"]
         tmp = out + f".{os.getpid()}.tmp"
         r = subprocess.run(base + ["-march=native", "-o", tmp], capture_output=True, text=True)
@@ -55,7 +60,11 @@ def build(force=False):
 def lib():
     global _lib
     if _lib is None:
-        h = C.CDLL(build())
+        if _stale(lib_path()):
+            with tempfile.TemporaryDirectory(prefix="nerrf_sage_oracle_") as d:
+                h = C.CDLL(build(out_dir=d))
+        else:
+            h = C.CDLL(lib_path())
         for n in ("nerrf_oracle_sage_layer", "nerrf_oracle_sage_aggregate", "nerrf_oracle_sage_node_head",
                   "nerrf_oracle_sage_forward", "nerrf_oracle_sage_threads"):
             getattr(h, n).restype = C.c_int

@@ -5,9 +5,11 @@
 * golden_hotpath.npz   seeded inputs + ORACLE outputs for GraphSAGE-T / LSTM / rewards / MCTS.
                        The reference ships no golden vectors for this path (SURVEY.md 8c): these
                        pin the oracle against drift and give the GPU tests a fixed target.
-* golden_m1_graph.npz  the temporal graph DERIVED from the reference's own LockBit trace
-                       benchmarks/m1/results/m1_trace.jsonl (+ m0) by nerrf_b200.graph (arrays only:
-                       CSR, features, labels).  /root/reference is not available on the GPU box.
+* golden_m1_graph.npz  the temporal graph DERIVED from the reference's own LockBit traces
+                       (benchmarks/m{0,1}/results/m{0,1}_trace.jsonl, stored here as m{0,1}_trace.jsonl)
+                       by nerrf_b200.graph (arrays only: CSR, features, labels); the encrypted files
+                       the reference lists (benchmarks/m{0,1}/results/file_list.txt) are stored here as
+                       m{0,1}_encrypted_files.txt.
 """
 import os
 import sys
@@ -46,26 +48,23 @@ def main():
     np.savez_compressed(os.path.join(HERE, "golden_hotpath.npz"), **out)
     print("golden_hotpath.npz:", {k: v.shape for k, v in out.items()})
 
-    ref = "/root/reference/benchmarks"
-    if os.path.isdir(ref):
-        tr = {}
-        for name in ("m0", "m1"):
-            gg = G.graph_from_jsonl(f"{ref}/{name}/results/{name}_trace.jsonl")
-            enc = sorted(l.split()[-1] for l in open(f"{ref}/{name}/results/file_list.txt") if ".lockbit3" in l)
-            names = gg.meta["names"]
-            # the same trace with OBSERVABLE features only (simulator annotations folded onto openat/write/rename):
-            # what ai/train.py trains on and what a wire-format trace of the same activity would give
-            go = G.graph_from_jsonl(f"{ref}/{name}/results/{name}_trace.jsonl", observable=True)
-            assert np.array_equal(go.rowptr, gg.rowptr) and np.array_equal(go.col, gg.col)
-            tr[f"{name}_x_obs"] = go.x
-            tr.update({f"{name}_rowptr": gg.rowptr, f"{name}_col": gg.col, f"{name}_ew": gg.ew, f"{name}_x": gg.x,
-                       f"{name}_label": gg.meta["label"], f"{name}_kind": gg.meta["node_kind"],
-                       f"{name}_size_mb": gg.meta["size_mb"],
-                       f"{name}_is_listed_encrypted": np.array([n in enc for n in names])})
-            print(name, gg.num_nodes, "nodes", gg.num_edges, "edges", int(gg.meta["label"].sum()), "attacked,", len(enc), "in file_list.txt")
-        np.savez_compressed(os.path.join(HERE, "golden_m1_graph.npz"), **tr)
-    else:
-        print("reference checkout not present: golden_m1_graph.npz not regenerated")
+    tr = {}
+    for name in ("m0", "m1"):
+        trace = os.path.join(HERE, f"{name}_trace.jsonl")
+        gg = G.graph_from_jsonl(trace)
+        enc = set(open(os.path.join(HERE, f"{name}_encrypted_files.txt")).read().split())
+        names = gg.meta["names"]
+        # the same trace with OBSERVABLE features only (simulator annotations folded onto openat/write/rename):
+        # what ai/train.py trains on and what a wire-format trace of the same activity would give
+        go = G.graph_from_jsonl(trace, observable=True)
+        assert np.array_equal(go.rowptr, gg.rowptr) and np.array_equal(go.col, gg.col)
+        tr[f"{name}_x_obs"] = go.x
+        tr.update({f"{name}_rowptr": gg.rowptr, f"{name}_col": gg.col, f"{name}_ew": gg.ew, f"{name}_x": gg.x,
+                   f"{name}_label": gg.meta["label"], f"{name}_kind": gg.meta["node_kind"],
+                   f"{name}_size_mb": gg.meta["size_mb"],
+                   f"{name}_is_listed_encrypted": np.array([n in enc for n in names])})
+        print(name, gg.num_nodes, "nodes", gg.num_edges, "edges", int(gg.meta["label"].sum()), "attacked,", len(enc), "listed encrypted")
+    np.savez_compressed(os.path.join(HERE, "golden_m1_graph.npz"), **tr)
 
 
 if __name__ == "__main__":

@@ -6,6 +6,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -14,8 +16,8 @@ def _run(*args):
                           timeout=600)
 
 
-def test_reference_arm_prints_the_contract_line():
-    r = _run("--impl", "reference", "--steps", "1", "--warmup", "0")
+def test_reference_arm_prints_the_contract_line(tmp_path):
+    r = _run("--impl", "reference", "--steps", "1", "--warmup", "0", "--dump-outputs", str(tmp_path))
     assert r.returncode == 0, r.stderr[-400:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -27,6 +29,12 @@ def test_reference_arm_prints_the_contract_line():
     cb = d["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and "sample" in cb
     assert d["e2e"] == {"value": d["value"], "unit": "edges/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+    # --dump-outputs: every node score and a fixed sample of embedding rows, float32, well under 64 MB
+    score, h = np.load(tmp_path / "score.npy"), np.load(tmp_path / "h_sample.npy")
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["h_sample.npy", "score.npy"]
+    assert score.dtype == h.dtype == np.float32 and score.shape == (1_000_000,) and h.shape == (32768, 128)
+    assert np.isfinite(score).all() and np.isfinite(h).all() and score.std() > 0 and h.std() > 0
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64 << 20
 
 
 def test_product_arm_needs_a_gpu():

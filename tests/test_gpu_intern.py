@@ -10,7 +10,7 @@ from nerrf_b200 import ingest, stream, trace_sim
 
 pytestmark = pytest.mark.gpu
 
-REF = "/root/reference/benchmarks"
+GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _same(cols, order=None, merge=True):
@@ -79,10 +79,10 @@ def test_random_paths_fuzz():
             _same(cols, rng.permutation(cols.n), merge)
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference traces not on this box")
 def test_reference_traces():
+    """The reference's own LockBit traces (benchmarks/m{0,1}/results/m{0,1}_trace.jsonl, stored under tests/golden/)."""
     for m in ("m0", "m1"):
-        ev = [json.loads(l) for l in open(f"{REF}/{m}/results/{m}_trace.jsonl")]
+        ev = [json.loads(l) for l in open(os.path.join(GOLD, f"{m}_trace.jsonl"))]
         _same(_cols(ev), None, True)
 
 
